@@ -141,7 +141,7 @@ def sample_flops(f, h, w, text_len=512):
 class CpuReference:
     """The reference's own modules on the host cores (fp32, F.scaled_dot_product_attention, all usable threads).
 
-    kind "reference": the UNMODIFIED reference staged under oracle/_ref (or /root/reference) through oracle/ref_runner.py —
+    kind "reference": the UNMODIFIED reference staged under oracle/_ref through oracle/ref_runner.py —
     one PCB DiTBlock, one VGGT frame Block and one IRGBlock at full 14B widths.  kind "port": oracle/fw_oracle.py, used only
     when no reference is staged.  Only this class and tests/ touch oracle/."""
 
@@ -332,6 +332,24 @@ def roofline_from_prof(prof, L, world, step_ms_total, sustained_peak, peak_src, 
             "share_of_step": tot / step_ms_total}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outs, out_dir):
+    """Write {name: tensor} as out_dir/<name>.npy in float32, DUMP_BYTES in all.  A tensor larger than its share is written as
+    the fixed sample (arange(n) * 2654435761 + 40503) mod numel of its flattened elements: the same positions on every run."""
+    import numpy as np
+    import torch
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // 4 // len(outs)
+    for name, t in outs.items():
+        t = t.detach()
+        if t.numel() > share:
+            t = t.reshape(-1)[(torch.arange(share, device=t.device) * 2654435761 + 40503) % t.numel()]
+        np.save(out_dir / f"{name}.npy", t.float().cpu().numpy())
+
+
 def _subprocess_json(cmd, timeout):
     """Run a helper process and parse the last stdout line as JSON ({"error": ...} on failure — a baseline leg must never
     take the measurement down with it)."""
@@ -350,7 +368,7 @@ def _subprocess_json(cmd, timeout):
 def gpu_reference_step(f, h, w, n_pcb, n_irg):
     """The UNMODIFIED reference on this same B200 (BASELINE.md §4): full-depth model under torch.autocast(bf16), one timed
     denoise step through its own joint_forward + scheduler (oracle/ref_runner.py `step`, separate process), after one warm-up."""
-    if not ((ROOT / "oracle" / "_ref" / "FantasyWorld").exists() or Path("/root/reference/FantasyWorld").exists()):
+    if not (ROOT / "oracle" / "_ref" / "FantasyWorld").exists():
         return {"unavailable": "reference not staged (python oracle/make_ref.py)"}
     out = _subprocess_json([sys.executable, str(ROOT / "oracle" / "ref_runner.py"), "step", "--device", "cuda", "--grid", str(f), str(h), str(w),
                             "--pcb", str(n_pcb), "--irg", str(n_irg), "--steps", "1", "--warmup", "1", "--modes", "bf16_fa2,bf16_sdpa"], timeout=1200)
@@ -467,6 +485,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t)
     sampler.stop_flag.set()
+    if args.dump_outputs and rank == 0:
+        dump_outputs({"latents": lat}, args.dump_outputs)        # what denoise_step returned in the last timed step
 
     # ---- e2e: host buffers through the public API ------------------------------------------------------------------------
     host = {k: v.cpu().pin_memory() for k, v in inp.items()}
@@ -598,6 +618,8 @@ def run_vggt_only(args):
     prof = fwb200.prof_disable()
     ms = e0.elapsed_time(e1)
     sampler.stop_flag.set()
+    if args.dump_outputs:
+        dump_outputs(pred, args.dump_outputs)                     # VGGT.forward's head outputs of the last timed step
     # e2e: patch tokens from pinned host memory, every head output read back
     outs = {k: torch.empty(v.shape, dtype=v.dtype).pin_memory() for k, v in pred.items()}
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -678,7 +700,14 @@ def main():
                     help="N=1: also time the unmodified reference (oracle/_ref) on the same GPU, in its own process")
     ap.add_argument("--cpu-budget", type=float, default=200.0, help="--impl reference: seconds for warmup + steps samples")
     ap.add_argument("--no-cpu-full", action="store_true", help="--impl reference: skip the extra full-token-count sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32, 64 MB in all; a larger "
+                         "output as a fixed sample of its elements), to compare two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.h is None:
         args.h, args.w = (45, 80) if args.workload == "wan22_720p" else (30, 52)
     protect_stdout()

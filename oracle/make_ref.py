@@ -29,7 +29,11 @@ TOP_LEVEL = ("inference_wan21.py", "inference_wan22.py", "utils.py")   # CLI bou
 def stage(force: bool = False) -> Path | None:
     """Copy FantasyWorld/**/*.py (+ the CLI files) from /root/reference to oracle/_ref.  Returns the destination, or None
     when the reference is absent (GPU box: the already-staged copy, if any, is used as is)."""
-    if not SRC.exists():
+    try:
+        present = SRC.is_dir()
+    except OSError:             # e.g. the reference sits in a directory this user may not enter
+        present = False
+    if not present:
         return DST if (DST / "MANIFEST.json").exists() else None
     files = sorted(p for p in (SRC / "FantasyWorld").rglob("*.py"))
     files += [SRC / n for n in TOP_LEVEL if (SRC / n).exists()]

@@ -1,4 +1,4 @@
-"""oracle/ref_runner.py — runs the UNMODIFIED reference (oracle/_ref or /root/reference, through tools/ref_shim.py) in its
+"""oracle/ref_runner.py — runs the UNMODIFIED reference (staged under oracle/_ref, through tools/ref_shim.py) in its
 own process, on the CPU or on the GPU box's B200.  TEST / BENCH INFRASTRUCTURE ONLY; nothing in the product path imports it.
 
 Why a separate process: the reference's package is called `FantasyWorld`, exactly like this repo's drop-in mirror, and it

@@ -11,7 +11,24 @@ GOLD = Path(__file__).resolve().parent / "golden"
 
 
 def gold(name):
-    return torch.load(GOLD / name, map_location="cpu", weights_only=False)
+    """A golden file; "parts" names further files whose tensors complete its "taps" (kept apart so no file exceeds 1 MB)."""
+    g = torch.load(GOLD / name, map_location="cpu", weights_only=False)
+    for part in g.pop("parts", []) if isinstance(g, dict) else []:
+        g.setdefault("taps", {}).update(torch.load(GOLD / part, map_location="cpu", weights_only=False))
+    return g
+
+
+def sample_index(numel, n=8192):
+    """Flat indices of a fixed sample of n elements out of numel (all of them when numel <= n): a multiplicative hash by a
+    prime, so the same positions are chosen on every machine and torch version."""
+    if numel <= n:
+        return torch.arange(numel)
+    return (torch.arange(n, dtype=torch.int64) * 2654435761 + 40503) % numel
+
+
+def take_sample(t, n=8192):
+    """The elements of `t` at sample_index(t.numel(), n), dtype kept."""
+    return t.detach().reshape(-1)[sample_index(t.numel(), n).to(t.device)].cpu()
 
 
 @functools.lru_cache(maxsize=1)

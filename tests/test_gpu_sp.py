@@ -80,7 +80,7 @@ def _worker(rank, world, port, ret):
         dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_sequence_parallel_2gpu_matches_single_gpu():
     import torch.multiprocessing as mp
     port = _free_port()

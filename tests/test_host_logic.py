@@ -171,7 +171,7 @@ def test_bench_reference_arm_prints_one_json_line():
               "dtype", "data", "config", "e2e", "cpu_baseline", "impl"):
         assert k in d, k
     assert d["impl"] == "reference" and d["metric"] == "denoise_steps_per_sec" and d["unit"] == "steps/s"
-    staged = (root / "oracle" / "_ref" / "FantasyWorld").exists() or Path("/root/reference/FantasyWorld").exists()
+    staged = (root / "oracle" / "_ref" / "FantasyWorld").exists()
     # the unmodified reference when it is staged (oracle/make_ref.py), the oracle port only as the fallback
     assert d["value"] > 0 and d["cpu_baseline"]["kind"] == ("reference" if staged else "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["ms_per_step"] == pytest.approx(1e3 * d["cpu_baseline"]["sample_seconds"])      # the measured sample, not the extrapolation

@@ -1,44 +1,47 @@
 """The reference runner (oracle/ref_runner.py: the UNMODIFIED reference in its own process) against the oracle on the CPU.
 
-This pins the plumbing the GPU parity tests rely on: the runner builds the reference with the per-key synthetic weights and
+This pins the plumbing the GPU parity goldens rely on: the runner builds the reference with the per-key synthetic weights and
 the seeded block inputs of fwb_synth, and must therefore reproduce what the oracle computes from the same state_dict and
-inputs (fp32, tolerance = summation order).  Skipped when no reference is staged (oracle/make_ref.py)."""
+inputs (fp32, tolerance = summation order).  The runner's output is the golden ref_runner_blocks_cpu.pt
+(tools/make_golden_ref_parity.py); the staging recipe that puts the reference next to the runner is checked on a scratch tree."""
 import json
-import subprocess
 import sys
 from pathlib import Path
 
-import pytest
 import torch
 
-from _common import rel_err, synth_state_dict
+from _common import gold, rel_err, synth_state_dict
 
 ROOT = Path(__file__).resolve().parent.parent
 
 
-def _available():
-    return Path("/root/reference/FantasyWorld").exists() or (ROOT / "oracle" / "_ref" / "FantasyWorld").exists()
-
-
-@pytest.mark.skipif(not _available(), reason="reference not staged (python oracle/make_ref.py)")
-def test_staged_reference_is_unmodified():
+def test_staged_reference_is_unmodified(tmp_path, monkeypatch):
     sys.path.insert(0, str(ROOT))
     from oracle import make_ref
-    if (ROOT / "oracle" / "_ref" / "MANIFEST.json").exists():
+    if (make_ref.DST / "MANIFEST.json").exists():
         assert make_ref.verify()
+    src, dst = tmp_path / "src", tmp_path / "dst"
+    (src / "FantasyWorld" / "fusion").mkdir(parents=True)
+    (src / "FantasyWorld" / "fusion" / "block.py").write_bytes(b"x = 1\n")
+    (src / "inference_wan21.py").write_bytes(b"import FantasyWorld\n")
+    monkeypatch.setattr(make_ref, "SRC", src)
+    monkeypatch.setattr(make_ref, "DST", dst)
+    assert make_ref.stage() == dst and make_ref.verify()
+    assert (dst / "FantasyWorld" / "fusion" / "block.py").read_bytes() == b"x = 1\n"
+    assert sorted(json.loads((dst / "MANIFEST.json").read_text())["files"]) == ["FantasyWorld/fusion/block.py", "inference_wan21.py"]
+    (dst / "inference_wan21.py").write_bytes(b"import FantasyWorld  # edited\n")
+    assert not make_ref.verify()
+    monkeypatch.setattr(make_ref, "SRC", tmp_path / "absent")
+    assert make_ref.stage() == dst            # no source: the copy already staged is used as is
 
 
-@pytest.mark.skipif(not _available(), reason="reference not staged (python oracle/make_ref.py)")
-def test_runner_blocks_match_oracle_fp32(tmp_path):
+def test_runner_blocks_match_oracle_fp32():
     from fwb_synth import synth_block_inputs
     from oracle import fw_oracle as O
     f, h, w, text_len = 1, 4, 4, 64
-    r = subprocess.run([sys.executable, str(ROOT / "oracle" / "ref_runner.py"), "blocks", "--device", "cpu", "--grid", str(f), str(h), str(w),
-                        "--text-len", str(text_len), "--modes", "fp32", "--out", str(tmp_path)], capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stderr[-2000:]
-    rep = json.loads(r.stdout.strip().splitlines()[-1])
-    assert rep["modes"]["fp32"]["dit_attention_backend"] == "F.scaled_dot_product_attention"
-    ref = torch.load(tmp_path / "blocks_fp32.pt")
+    ref = gold("ref_runner_blocks_cpu.pt")
+    assert ref["report"]["grid"] == [f, h, w]
+    assert ref["report"]["modes"]["fp32"]["dit_attention_backend"] == "F.scaled_dot_product_attention"
     sd = {k: v.to(torch.bfloat16).float() for k, v in synth_state_dict().items()}      # the fp32 mode runs on bf16-valued weights
     inp = synth_block_inputs(f, h, w, text_len)
     tab, tab_d, tab_a = O.rope_table_3d(128, f, h, w), O.rope_table_3d(96, f, h, w), O.rope_table_3d_with_extra(96, f, h, w, 5)

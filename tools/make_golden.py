@@ -95,8 +95,11 @@ def main():
                                     plucker_context_lens=lens, return_prediction=True)
     for hk in hooks:
         hk.remove()
-    torch.save({"out": out.clone(), "pred": {k: v.clone() for k, v in pred.items()}, "taps": taps, "grid": (F, H, W),
-                "text_len": TEXT_LEN, "timestep": TIMESTEP, "head_layer_idx": HEAD_LAYER_IDX}, GOLD / "joint_forward.pt")
+    parts = {"after_pcb": "joint_forward_after_pcb.pt", "after_irg_x": "joint_forward_after_irg_x.pt"}     # each file under 1 MB
+    for k, name in parts.items():
+        torch.save({k: taps.pop(k)}, GOLD / name)
+    torch.save({"out": out.clone(), "pred": {k: v.clone() for k, v in pred.items()}, "taps": taps, "parts": list(parts.values()),
+                "grid": (F, H, W), "text_len": TEXT_LEN, "timestep": TIMESTEP, "head_layer_idx": HEAD_LAYER_IDX}, GOLD / "joint_forward.pt")
     print("joint_forward done", out.abs().mean().item(), {k: tuple(v.shape) for k, v in pred.items()})
 
     # ---------------- one denoise step (CFG 5.0) ----------------

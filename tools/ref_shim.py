@@ -8,8 +8,7 @@ CPU baseline (oracle/ref_runner.py, always in its OWN process: the reference's p
 this repo's mirror, so the two never share an interpreter).  Lives under tools/ (it is an import helper for the reference, not part
 of the oracle): the golden generators import it directly, oracle/ref_runner.py loads it by path.
 
-Where the reference comes from: /root/reference in the build container; on the GPU box (no /root/reference) the byte-for-byte
-copy staged by oracle/make_ref.py under oracle/_ref/ (git-ignored, shipped by gpurun).
+Where the reference comes from: the byte-for-byte copy staged by oracle/make_ref.py under oracle/_ref/ (git-ignored).
 """
 from __future__ import annotations
 
@@ -22,8 +21,7 @@ import torch.nn as nn
 
 from pathlib import Path
 
-_STAGED = Path(__file__).resolve().parent.parent / "oracle" / "_ref"
-REF_ROOT = "/root/reference" if Path("/root/reference/FantasyWorld").exists() else str(_STAGED)
+REF_ROOT = str(Path(__file__).resolve().parent.parent / "oracle" / "_ref")
 
 
 def reference_available() -> bool:
