@@ -112,7 +112,8 @@ class CrossAttentionAdapterProcessor(nn.Module):
         return w0, b0, w2, E.f32(l2, "b", l2.bias)
 
     def _adaln(self, o, plucker_fea):
-        """o [L, C] bf16 (text+CLIP attention output) -> o + shift."""
+        """o [B*L, C] bf16 (text+CLIP attention output) -> o + shift; plucker_fea [B, L, 2048].  As in the reference, one
+        all-zero test covers the whole batch: a batch with one all-zero sample still shifts every sample."""
         all_zero, p1 = self._plucker(plucker_fea)
         if all_zero:
             return o
@@ -133,8 +134,8 @@ class CrossAttentionAdapterProcessor(nn.Module):
     def __call__(self, attn: nn.Module, x: torch.Tensor, y: torch.Tensor, plucker_fea: torch.Tensor = None,
                  plucker_context_lens: torch.Tensor = None, pose_scale: float = 1.0):
         b, s, c = x.shape
-        assert b == 1 and pose_scale == 1.0
-        o = E.dit_cross_attn_core(attn, E.as_bf16(x).reshape(s, c), y)
+        assert pose_scale == 1.0, "pose_scale != 1 is not used by the reference sampler"
+        o = E.dit_cross_attn_core(attn, E.as_bf16(x).reshape(b * s, c), y)
         if plucker_fea is not None:
             o = self._adaln(o, plucker_fea)
         return E.lin(o, attn.o, round_flags=ops.ROUND_AFTER_BIAS).view(b, s, c)

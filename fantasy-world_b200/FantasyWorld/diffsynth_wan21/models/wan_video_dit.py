@@ -79,9 +79,7 @@ def rope_apply(x, freqs, num_heads):
     b, s, c = x.shape
     d = c // num_heads
     y = E.as_bf16(x).clone().view(b * s, c)
-    cs = E.complex_to_cos_sin(freqs, x.device)
-    if b > 1:
-        cs = cs.repeat(b, 1, 1)
+    cs = E.complex_to_cos_sin(freqs, x.device)          # [s] rows, applied to every sample
     ops.rmsnorm_rope_(y, cos_sin=cs, head_dim=d)
     return y.view(b, s, c).to(x.dtype)
 
@@ -129,15 +127,13 @@ class SelfAttention(nn.Module):
 
     def forward(self, x, freqs):
         b, s, c = x.shape
-        assert b == 1, "fused path: batch 1"
-        h = E.as_bf16(x).reshape(s, c)
+        h = E.as_bf16(x).reshape(b * s, c)
         cs = E.complex_to_cos_sin(freqs, x.device)
-        L = h.shape[0]
         q, k, v = E.lin(h, self.q), E.lin(h, self.k), E.lin(h, self.v)
         ops.rmsnorm_rope_(q, w=E.f32(self.norm_q, "w", self.norm_q.weight), eps=self.norm_q.eps, cos_sin=cs, head_dim=self.head_dim)
         ops.rmsnorm_rope_(k, w=E.f32(self.norm_k, "w", self.norm_k.weight), eps=self.norm_k.eps, cos_sin=cs, head_dim=self.head_dim)
-        o = ops.attention(q.view(1, L, self.num_heads, -1), k.view(1, L, self.num_heads, -1), v.view(1, L, self.num_heads, -1))
-        return E.lin(o.view(L, c), self.o, round_flags=ops.ROUND_AFTER_BIAS).view(b, s, c)
+        o = ops.attention(q.view(b, s, self.num_heads, -1), k.view(b, s, self.num_heads, -1), v.view(b, s, self.num_heads, -1))
+        return E.lin(o.view(b * s, c), self.o, round_flags=ops.ROUND_AFTER_BIAS).view(b, s, c)
 
 
 class CrossAttentionProcessor:
@@ -145,7 +141,7 @@ class CrossAttentionProcessor:
 
     def __call__(self, attn, x: torch.Tensor, y: torch.Tensor):
         b, s, c = x.shape
-        o = E.dit_cross_attn_core(attn, E.as_bf16(x).reshape(s, c), y)
+        o = E.dit_cross_attn_core(attn, E.as_bf16(x).reshape(b * s, c), y)
         return E.lin(o, attn.o, round_flags=ops.ROUND_AFTER_BIAS).view(b, s, c)
 
     # fused-block hook: returns o(o_attn) + resid without materialising the intermediate
@@ -217,8 +213,7 @@ class DiTBlock(nn.Module):
     def forward(self, x, context=None, t_mod=None, freqs=None, *, return_partial: bool = False,
                 run_remaining: bool = False, modifiers: tuple | None = None, **kwargs):
         b, s, c = x.shape
-        assert b == 1, "fused path handles batch 1 (the reference sampler's batch)"
-        xs = E.as_bf16(x).reshape(s, c)
+        xs = E.as_bf16(x).reshape(b * s, c)
         if run_remaining:
             assert modifiers is not None, "modifiers must provide"
             return E.dit_ffn(self, xs, modifiers).view(b, s, c)
@@ -229,7 +224,7 @@ class DiTBlock(nn.Module):
             r0, r1 = E.SP.layout.video_range(E.SP.rank)
             cs = cs[r0:r1]
         h = ops.ln_modulate(xs, eps=self.norm1.eps, mul=mods["mul_msa"], add=mods["shift_msa"])
-        xs = E.dit_self_attn(self.self_attn, h, cs, xs, mods["gate_msa"])
+        xs = E.dit_self_attn(self.self_attn, h, cs, xs, mods["gate_msa"], n_batch=b)
         n3 = ops.ln_modulate(xs, eps=self.norm3.eps, w=E.f32(self.norm3, "w", self.norm3.weight),
                              b=E.f32(self.norm3, "b", self.norm3.bias))
         proc = self.cross_attn.processor
@@ -282,11 +277,11 @@ class Head(nn.Module):
 
     def forward(self, x, t_mod):
         b, s, c = x.shape
-        assert b == 1
-        m = self.modulation.to(dtype=t_mod.dtype, device=t_mod.device) + t_mod.reshape(1, -1, c)  # [1,2,C]
+        t_mod = E.shared_rows(t_mod.reshape(-1, 1, c), "Head")                                      # shared timestep
+        m = self.modulation.to(dtype=t_mod.dtype, device=t_mod.device) + t_mod  # [1,2,C]
         shift = m[0, 0].float().contiguous()
         mul = (1 + m[0, 1]).float().contiguous()
-        h = ops.ln_modulate(E.as_bf16(x).reshape(s, c), eps=self.norm.eps, mul=mul, add=shift)
+        h = ops.ln_modulate(E.as_bf16(x).reshape(b * s, c), eps=self.norm.eps, mul=mul, add=shift)
         return E.lin(h, self.head, round_flags=ops.ROUND_AFTER_BIAS).view(b, s, -1)
 
 

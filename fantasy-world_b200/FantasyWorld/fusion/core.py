@@ -30,10 +30,46 @@ class FusionCore(nn.Module):
         self.sp = self.cfgp.sp
         return self.cfgp
 
-    def _cfg_forwards(self, latents, t, context_pos, context_neg, kw, return_prediction):
+    # per-sample keyword inputs of joint_forward (batch dimension first); everything else is shared by the batch
+    PER_SAMPLE_KW = ("clip_feature", "y", "plucker_fea", "control_camera_latents_input", "camera_token")
+
+    def check_batch(self, latents, context_pos, context_neg, kw, batch_cfg=False):
+        """Batch size of a sampler call, validated: every per-sample input has the batch size of `latents` (no implicit
+        broadcasting), and a batch > 1 or `batch_cfg` is refused under sequence or CFG parallelism."""
+        b = latents.shape[0]
+        named = [("context_pos", context_pos), ("context_neg", context_neg)] + [(k, kw.get(k)) for k in self.PER_SAMPLE_KW]
+        for name, v in named:
+            if v is not None and v.shape[0] != b:
+                raise ValueError(f"{name} has batch {v.shape[0]}, latents have batch {b}: every per-sample input needs the same batch")
+        parallel = self.cfgp is not None or (self.sp is not None and self.sp.world > 1)
+        if batch_cfg and parallel:
+            raise ValueError("batch_cfg=True runs both CFG forwards as one batch on one GPU; it cannot be combined with "
+                             "enable_cfg_parallel() or sequence parallelism (model.sp)")
+        if b > 1 and parallel:
+            raise ValueError(f"a batch of {b} is not supported under sequence or CFG parallelism: run batch 1 per call")
+        return b
+
+    def _cat_cached(self, *ts):
+        """torch.cat(ts) of loop-invariant inputs, cached per tensor tuple (stable identity keeps the context / K-V caches warm)."""
+        cache = self.__dict__.get("_fwb_cat")
+        if cache is None:
+            cache = self.__dict__["_fwb_cat"] = E.IdCache(8)
+        return cache.get(ts, None, lambda: torch.cat(ts))
+
+    def _cfg_forwards(self, latents, t, context_pos, context_neg, kw, return_prediction, batch_cfg=False):
         """(pred_pos, pred_neg, prediction) of one step.  Serial: both forwards here (reference order, model_wan21.py:295-317).
         CFG-parallel: this rank evaluates only its half's forward and the halves swap predictions; the geometry-head
-        prediction exists on the conditional half only (the reference takes it from the conditional pass)."""
+        prediction exists on the conditional half only (the reference takes it from the conditional pass).
+        batch_cfg: ONE forward of batch 2B over cat([latents, latents]) with cat([context_pos, context_neg]); the two
+        predictions are the contiguous halves of its output and the head prediction comes from the conditional half."""
+        b = self.check_batch(latents, context_pos, context_neg, kw, batch_cfg)
+        if batch_cfg:
+            kw2 = {k: (self._cat_cached(v, v) if k in self.PER_SAMPLE_KW and v is not None else v) for k, v in kw.items()}
+            out, pred = self.joint_forward(torch.cat([latents, latents]), timestep=t, context=self._cat_cached(context_pos, context_neg),
+                                           return_prediction=return_prediction, **kw2)
+            if pred is not None:
+                pred = {k: v[:b] for k, v in pred.items()}
+            return out[:b], out[b:], pred
         if self.cfgp is None:
             pred_pos, pred = self.joint_forward(latents, timestep=t, context=context_pos, return_prediction=return_prediction, **kw)
             pred_neg, _ = self.joint_forward(latents, timestep=t, context=context_neg, **kw)
@@ -95,23 +131,29 @@ class FusionCore(nn.Module):
             cache = self.__dict__["_fwb_ctrl"] = E.IdCache(2)
 
         def build():
-            yc = dit.control_adapter(control)                    # [b, dim, f, h, w]
-            assert yc.shape[0] == 1
-            return E.as_bf16(yc[0].permute(1, 2, 3, 0).reshape(-1, yc.shape[1])).contiguous()
+            yc = dit.control_adapter(control)                    # [b, dim, f, h, w] -> [(b f h w), dim]
+            return E.as_bf16(yc.permute(0, 2, 3, 4, 1).reshape(-1, yc.shape[1])).contiguous()
 
         return cache.get((control, dit.control_adapter.conv.weight), None, build)
 
     # ---- the shared forward -----------------------------------------------------------------------------------------------
     def _joint_core(self, x, timestep, ctx, block_kw, plucker_fea=None, control=None, camera_token=None, uncond=False,
                     return_prediction=False):
-        """x: the concatenated latent [1, C_in, F, H, W]; ctx: embedded context [1, n_ctx, dim].  Single GPU when self.sp is
-        None (or world 1), otherwise token-sharded (SURVEY §8e): video rows L/P per rank, frame-aligned geometry shards, one
-        all-gather of packed K|V per attention, one gather of the projected tokens and one of the head output per forward."""
+        """x: the concatenated latent [B, C_in, F, H, W]; ctx: embedded context [B, n_ctx, dim].  Single GPU when self.sp is
+        None (or world 1), otherwise token-sharded (SURVEY §8e, batch 1 only): video rows L/P per rank, frame-aligned geometry
+        shards, one all-gather of packed K|V per attention, one gather of the projected tokens and one of the head output per
+        forward.  At batch B every sample has its own latents, context and camera inputs and all share the timestep; each
+        sample's tokens attend only to its own (B*L token rows, [B, L, H, D] attention views)."""
         sp = self.sp if (self.sp is not None and self.sp.world > 1) else None
         dit, vggt, agg = self.pipe.dit, self.vggt, self.vggt.aggregator
-        t, t_mod = dit.embed_time(timestep)
         b, cin, F_, H_, W_ = x.shape
-        assert b == 1
+        timestep = E.shared_timestep(timestep, b)
+        if sp is not None and b > 1:
+            raise ValueError(f"a batch of {b} is not supported under sequence parallelism")
+        for name, v in (("context", ctx), ("plucker_fea", plucker_fea), ("control_camera_latents_input", control)):
+            if v is not None and v.shape[0] != b:
+                raise ValueError(f"{name} has batch {v.shape[0]}, the latents have batch {b}")
+        t, t_mod = dit.embed_time(timestep)
         pf, ph, pw = dit.patch_size
         f, h, w = F_ // pf, H_ // ph, W_ // pw
         L = f * h * w
@@ -123,11 +165,13 @@ class FusionCore(nn.Module):
         else:
             r0, r1, f0, f1 = 0, L, 0, f
         # patchify: Conv3d(k = s = patch) as a GEMM over unfolded patches, only this rank's rows (ref: wan_video_dit.py:424-435)
-        cols = E.as_bf16(x).view(b, cin, f, pf, h, ph, w, pw).permute(0, 2, 4, 6, 1, 3, 5, 7).reshape(L, cin * pf * ph * pw)
+        cols = E.as_bf16(x).view(b, cin, f, pf, h, ph, w, pw).permute(0, 2, 4, 6, 1, 3, 5, 7).reshape(b * L, cin * pf * ph * pw)
         resid = None
         if control is not None and dit.control_adapter is not None:
-            resid = self._control_tokens(control)[r0:r1]
-        xl = E.lin(cols[r0:r1].contiguous(), dit.patch_embedding, resid=resid, round_flags=ops.ROUND_AFTER_BIAS).unsqueeze(0)
+            resid = self._control_tokens(control)
+            resid = resid[r0:r1] if sp is not None else resid
+        cols = cols[r0:r1] if sp is not None else cols
+        xl = E.lin(cols.contiguous(), dit.patch_embedding, resid=resid, round_flags=ops.ROUND_AFTER_BIAS).view(b, -1, dit.dim)
         freqs, freqs_bi_dit, freqs_bi_agg = self.rope_tables(f, h, w, xl.device)
         kw = dict(block_kw)
         if plucker_fea is not None:
@@ -138,10 +182,10 @@ class FusionCore(nn.Module):
             for i in range(self.start_index):                                   # Preconditioning Blocks
                 xl = dit.blocks[i](xl, ctx, t_mod, freqs, **kw)
             # 5120 -> 1024 projection on local rows (then, under SP, one gather so that every rank can pick its frames)
-            proj = vggt.project_tokens(xl)[0]
+            proj = vggt.project_tokens(xl)
             if sp is not None:
-                proj = sp.all_gather_rows(proj, lay.video_rows)
-            patch_all = proj.view(1, f, h, w, -1)
+                proj = sp.all_gather_rows(proj[0], lay.video_rows)
+            patch_all = proj.view(b, f, h, w, -1)
             e0 = vggt.time_modulation(timestep)
             if sp is not None:
                 tokens, pos = agg._process_aggregator_input(patch_all[:, f0:f1], None, frame_range=(f0, f1))
@@ -158,7 +202,7 @@ class FusionCore(nn.Module):
             frame_idx = global_idx = 0
             output_list = []
             for i in range(n_layers):
-                tokens, frame_idx, frame_inter = agg._process_frame_attention(tokens, 1, S, P, C, frame_idx, pos=pos, e0=e0)
+                tokens, frame_idx, frame_inter = agg._process_frame_attention(tokens, b, S, P, C, frame_idx, pos=pos, e0=e0)
                 if i in self.cross_attention_list:
                     xl, tokens, global_inter = self.IRGBlock[i](x_dit=xl, x_agg=tokens, context=ctx, t_mod=t_mod, freqs=freqs,
                                                                 freqs_dit=freqs_bi_dit, freqs_agg=freqs_bi_agg, pos=pos, e0=e0,
@@ -167,7 +211,7 @@ class FusionCore(nn.Module):
                 else:
                     assert sp is None, "sequence parallel path expects every post-PCB block to be an IRG block"
                     xl = dit.blocks[i + self.start_index](xl, ctx, t_mod, freqs, **kw)
-                    tokens, global_idx, global_inter = agg._process_global_attention(tokens, 1, S, P, C, global_idx, pos=pos, e0=e0)
+                    tokens, global_idx, global_inter = agg._process_global_attention(tokens, b, S, P, C, global_idx, pos=pos, e0=e0)
                 if return_prediction:  # only the last step consumes these 2C-wide intermediates (ref: :208-212, :217-222)
                     if sp is None:
                         output_list.extend(torch.cat([a, b_], dim=-1) for a, b_ in zip(frame_inter, global_inter))
@@ -182,6 +226,10 @@ class FusionCore(nn.Module):
         if sp is not None:
             out = sp.all_gather_rows(out[0].contiguous(), lay.video_rows).unsqueeze(0)
         out = dit.unpatchify(out, (f, h, w))
-        if return_prediction:
+        if not return_prediction:
+            return out, None
+        if b == 1:
             return out, vggt._head_predction(patch_all, agg.patch_start_idx, output_list)
-        return out, None
+        # the heads run per sample: their convolutions then see the batch-1 shapes of a single call
+        preds = [vggt._head_predction(patch_all[i:i + 1], agg.patch_start_idx, [o[i:i + 1] for o in output_list]) for i in range(b)]
+        return out, {k: torch.cat([p[k] for p in preds]) for k in preds[0]}

@@ -65,18 +65,22 @@ class CrossModalityBiAttentionBlock(nn.Module):
         x1, x2 = xs
         if attention_masks[0] is not None or attention_masks[1] is not None:
             raise NotImplementedError('attention mask is currently unsupported for video-audio cross attention')
-        assert x1.shape[0] == 1 and x2.shape[0] == 1, "fused path: batch 1"
-        a = E.as_bf16(x1)[0]
-        g = x2[0] if x2.dtype in (torch.float32, torch.bfloat16) else x2[0].float()
+        B = x1.shape[0]
+        if x2.shape[0] != B:
+            raise ValueError(f"video batch {B} != geometry batch {x2.shape[0]}")
+        a = E.as_bf16(x1).reshape(-1, x1.shape[-1])
+        g = x2.reshape(-1, x2.shape[-1])
+        if g.dtype not in (torch.float32, torch.bfloat16):
+            g = g.float()
         cs_dit, cs_agg = E.complex_to_cos_sin(freqs_dit, x1.device), E.complex_to_cos_sin(freqs_agg, x1.device)
-        if E.SP is not None:   # sequence parallel: both streams hold this rank's rows only
+        if E.SP is not None:   # sequence parallel (batch 1): both streams hold this rank's rows only
             lay, rk = E.SP.layout, E.SP.rank
             if cs_dit.shape[0] != a.shape[0]:
                 cs_dit = cs_dit[slice(*lay.video_range(rk))]
             if cs_agg.shape[0] != g.shape[0]:
                 cs_agg = cs_agg[slice(*lay.geo_range(rk))]
-        a, g = E.bicross(self, a, g, cs_dit, cs_agg)
-        return a.unsqueeze(0), g.unsqueeze(0)
+        a, g = E.bicross(self, a, g, cs_dit, cs_agg, n_batch=B)
+        return a.view(B, -1, a.shape[-1]), g.view(B, -1, g.shape[-1])
 
 
 class IRGBlock(nn.Module):

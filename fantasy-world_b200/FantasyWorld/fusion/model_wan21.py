@@ -92,9 +92,12 @@ class FantasyWorldFusionModel(FusionCore):
                        clip_feature: Optional[torch.Tensor] = None, y: Optional[torch.Tensor] = None,
                        use_gradient_checkpointing: bool = False, camera_token=None, height=480, width=832, num_frames=81,
                        num_inference_steps=50, cfg_scale=5.0, seed=None, device="cuda", plucker_embedding=None,
-                       geo_prior=None, latents: Optional[torch.Tensor] = None, **kwargs):
+                       geo_prior=None, latents: Optional[torch.Tensor] = None, batch_cfg: bool = False, **kwargs):
         """50-step CFG flow-matching sampler.  ref: model_wan21.py:227-324.  `latents` (extension) injects the initial
-        noise instead of drawing it (GPU RNG streams are not reproducible across devices, SURVEY Appendix D-6)."""
+        noise instead of drawing it (GPU RNG streams are not reproducible across devices, SURVEY Appendix D-6).
+        Batch (extension): the batch is that of `latents`, or of `context_pos` when the noise is drawn here; every
+        per-sample input (contexts, clip_feature, y, plucker_embedding, geo_prior) must have that batch.  `batch_cfg`: see
+        denoise_step."""
         pipe = self.pipe
         if num_frames % 4 != 1:
             num_frames = (num_frames + 2) // 4 * 4 + 1
@@ -102,8 +105,8 @@ class FantasyWorldFusionModel(FusionCore):
         if latents is None:
             if seed is not None:
                 torch.manual_seed(1024)
-            noise = pipe.generate_noise((1, 16, (num_frames - 1) // 4 + 1, height // 8, width // 8), seed=seed, device=device,
-                                        dtype=torch.float32)
+            noise = pipe.generate_noise((context_pos.shape[0], 16, (num_frames - 1) // 4 + 1, height // 8, width // 8), seed=seed,
+                                        device=device, dtype=torch.float32)
             latents = noise.to(dtype=pipe.torch_dtype, device=pipe.device)
         latents = latents.to(dtype=torch.bfloat16, device=pipe.device).contiguous().clone()
 
@@ -129,7 +132,7 @@ class FantasyWorldFusionModel(FusionCore):
             latents, pred = self.denoise_step(latents, step, context_pos, context_neg, clip_feature=clip_feature, y=y,
                                               camera_token=camera_token, plucker_fea=plucker_fea,
                                               plucker_context_lens=plucker_context_lens, cfg_scale=cfg_scale,
-                                              return_prediction=(step == num_inference_steps - 1), **extra)
+                                              return_prediction=(step == num_inference_steps - 1), batch_cfg=batch_cfg, **extra)
             if pred is not None:
                 final_prediction = pred
         return latents, final_prediction
@@ -138,11 +141,13 @@ class FantasyWorldFusionModel(FusionCore):
     def denoise_step(self, latents: torch.Tensor, step: int, context_pos: torch.Tensor, context_neg: Optional[torch.Tensor] = None,
                      clip_feature: Optional[torch.Tensor] = None, y: Optional[torch.Tensor] = None, camera_token=None,
                      plucker_fea: Optional[torch.Tensor] = None, plucker_context_lens: Optional[torch.Tensor] = None,
-                     cfg_scale: float = 5.0, return_prediction: bool = False, **extra):
+                     cfg_scale: float = 5.0, return_prediction: bool = False, batch_cfg: bool = False, **extra):
         """One iteration of the sampler loop (ref: model_wan21.py:289-322): conditional + unconditional joint_forward,
         classifier-free guidance and the flow-matching Euler update (fused in fwb_cfg_euler_step).  `latents` may live on
         the host (pinned): it is copied to the device here; the updated latents are returned on the device.
-        Uses the schedule set by `self.pipe.scheduler.set_timesteps`."""
+        Uses the schedule set by `self.pipe.scheduler.set_timesteps`.
+        latents [B, ...] with per-sample contexts [B, ...] (one shared timestep).  batch_cfg=True evaluates the conditional
+        and unconditional forwards as ONE forward of batch 2B (same results; off by default, see DESIGN.md §1 "Batch")."""
         pipe, sched = self.pipe, self.pipe.scheduler
         dev = pipe.device
         if latents.device.type != "cuda":
@@ -154,10 +159,12 @@ class FantasyWorldFusionModel(FusionCore):
                   plucker_fea=plucker_fea, plucker_context_lens=plucker_context_lens)
         dsigma = sched.dsigma(t_host)
         if cfg_scale != 1.0 and context_neg is not None:
-            pred_pos, pred_neg, pred = self._cfg_forwards(latents, t, context_pos, context_neg, {**kw, **extra}, return_prediction)
+            pred_pos, pred_neg, pred = self._cfg_forwards(latents, t, context_pos, context_neg, {**kw, **extra}, return_prediction,
+                                                          batch_cfg=batch_cfg)
             ops.cfg_euler_step_(latents, pred_pos.contiguous(), pred_neg.contiguous(), cfg_scale, dsigma)
         else:
             assert self.cfgp is None, "CFG parallelism needs cfg_scale != 1 and a negative context"
+            self.check_batch(latents, context_pos, None, kw)
             pred_pos, pred = self.joint_forward(latents, timestep=t, context=context_pos, return_prediction=return_prediction, **kw, **extra)
             ops.cfg_euler_step_(latents, pred_pos.contiguous(), pred_pos.contiguous(), 1.0, dsigma)
         return latents, pred

@@ -133,18 +133,20 @@ class FantasyWorldFusionModel(FusionCore):
 @torch.no_grad()
 def denoise_step_experts(model_high: FantasyWorldFusionModel, model_low: FantasyWorldFusionModel, latents, step, context_pos,
                          context_neg, y, control_camera_latents_input, timestep_boundary=900.0, cfg_scale=5.0,
-                         return_prediction=False):
+                         return_prediction=False, batch_cfg=False):
     """One iteration of inference_wan22.py's loop (ref: inference_wan22.py:229-280): pick the high-noise or low-noise expert
-    by timestep, two forwards (CFG), fused guidance + Euler update."""
+    by timestep, two forwards (CFG), fused guidance + Euler update.  Batched latents / contexts and `batch_cfg` as in the
+    Wan2.1 model's denoise_step."""
     sched = model_high.pipe.scheduler
     t_host = sched.timesteps[step]
     model = model_high if select_high_noise_expert(t_host, timestep_boundary) else model_low
     t = t_host.unsqueeze(0).to(dtype=torch.bfloat16, device=latents.device)
     kw = dict(y=y, use_gradient_checkpointing=False, camera_token=None, control_camera_latents_input=control_camera_latents_input)
     if cfg_scale != 1.0 and context_neg is not None:
-        pos, neg, pred = model._cfg_forwards(latents, t, context_pos, context_neg, kw, return_prediction)   # serial or CFG-parallel
+        pos, neg, pred = model._cfg_forwards(latents, t, context_pos, context_neg, kw, return_prediction, batch_cfg=batch_cfg)
         ops.cfg_euler_step_(latents, pos.contiguous(), neg.contiguous(), cfg_scale, sched.dsigma(t_host))
     else:
+        model.check_batch(latents, context_pos, None, kw)
         pos, pred = model.joint_forward(latents, timestep=t, context=context_pos, return_prediction=return_prediction, **kw)
         ops.cfg_euler_step_(latents, pos.contiguous(), pos.contiguous(), 1.0, sched.dsigma(t_host))
     return latents, pred

@@ -76,21 +76,25 @@ class Aggregator(nn.Module):
             cam = self.camera_token[0, slot].to(flat.dtype)       # [T, 1, C]
             reg = self.register_token[0, slot].to(flat.dtype)     # [T, 4, C]
         tokens = torch.cat([cam, reg, flat], dim=1)
-        return tokens, self._positions(B * T, gh, gw, flat.device)
+        return tokens, self._positions(B * T, gh, gw, flat.device, batch=B)
 
-    def _positions(self, n, gh, gw, device):
+    def _positions(self, n, gh, gw, device, batch=1):
         """int64 [n, 5 + gh*gw, 2]; loop-invariant, so built once per (n, gh, gw) and reused (stable identity lets the
-        RoPE tables derived from it be cached too)."""
+        RoPE tables derived from it be cached too).  At batch > 1 every sample has the same positions: the tensor is marked
+        with the rows of one sample (`_fwb_period`), so the RoPE tables are built for one sample and shared."""
         if self.rope is None:
             return None
         cache = self.__dict__.setdefault("_pos_cache", {})
-        key = (n, gh, gw, str(device))
+        key = (n, gh, gw, str(device), batch)
         if key not in cache:
             pos = self.position_getter(n, gh, gw, device=device)
             if self.patch_start_idx > 0:
                 special = torch.zeros(n, self.patch_start_idx, 2, device=device, dtype=pos.dtype)
                 pos = torch.cat([special, pos + 1], dim=1)
-            cache[key] = pos.contiguous()
+            pos = pos.contiguous()
+            if batch > 1:
+                pos._fwb_period = (n // batch) * pos.shape[1]
+            cache[key] = pos
         return cache[key]
 
     # -- attention drivers ---------------------------------------------------------------------------------------------

@@ -7,6 +7,8 @@
 //                                                                         fusion/layer/block.py:545-550
 //   fwb_ln64_rope2d     per-head LayerNorm(64) + 2-D rotate-half RoPE on the q and k thirds of a packed qkv buffer
 //                                                                         vggt/layers/attention.py:52-58 ; vggt/layers/rope.py:133-188
+//   *_periodic          the same two RoPE kernels reading table row (row % table_rows): at batch B the token rows are B*L
+//                       while the RoPE table is per position (L rows), so one table serves every sample
 //   fwb_cfg_euler_step  latents += (neg + s*(pos-neg)) * dsigma           fusion/model_wan21.py:318-322 ; flow_match.py:43-53
 //
 // All are bandwidth bound: one pass over the row, 128-bit loads/stores, fp32 statistics with warp-shuffle reductions.
@@ -180,7 +182,7 @@ ln_modulate_kernel(const void* __restrict__ x, long long ldx, int rows, int C, f
 template <int CHUNKS>
 __global__ void __launch_bounds__(kRowThreads)
 rmsnorm_rope_kernel(__nv_bfloat16* __restrict__ x, long long ldx, int rows, int C, const float* __restrict__ w,
-                    float eps, const float2* __restrict__ cs, int head_dim) {
+                    float eps, const float2* __restrict__ cs, int table_rows, int head_dim) {
   // persistent rows with the next row prefetched, as ln_modulate_kernel (in place: a row is only ever touched by one CTA)
   __shared__ float red[2][4];           // one reduction per row: alternate by row (see block_sum)
   int flip = 0;
@@ -226,7 +228,7 @@ rmsnorm_rope_kernel(__nv_bfloat16* __restrict__ x, long long ldx, int rows, int 
         }
         if (cs) {
           const int d0 = (c0 % head_dim) >> 1;  // first pair index inside the head
-          const float2* t = cs + (size_t)row * half + d0;
+          const float2* t = cs + (size_t)(row % table_rows) * half + d0;
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
             const float2 c = __ldg(t + j);  // (cos, sin)
@@ -251,7 +253,7 @@ rmsnorm_rope_kernel(__nv_bfloat16* __restrict__ x, long long ldx, int rows, int 
 __global__ void __launch_bounds__(256)
 ln64_rope2d_kernel(__nv_bfloat16* __restrict__ qkv, long long ld, int rows, int H, float eps,
                    const float* __restrict__ qw, const float* __restrict__ qb, const float* __restrict__ kw,
-                   const float* __restrict__ kb, const float* __restrict__ cosT, const float* __restrict__ sinT) {
+                   const float* __restrict__ kb, const float* __restrict__ cosT, const float* __restrict__ sinT, int table_rows) {
   const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long group = gid >> 3;  // (row, which in {q,k}, head)
   const int g = (int)(gid & 7);
@@ -302,8 +304,9 @@ ln64_rope2d_kernel(__nv_bfloat16* __restrict__ qkv, long long ld, int rows, int 
   for (int j = 0; j < 8; ++j) part[j] = __shfl_xor_sync(0xffffffffu, y[j], 2);
   if (active) {
     float cc[8], ss[8];
-    load8_f32(cosT + row * 64 + g * 8, cc);
-    load8_f32(sinT + row * 64 + g * 8, ss);
+    const long long trow = (int)row % table_rows;    // row < rows (int): 32-bit modulo
+    load8_f32(cosT + trow * 64 + g * 8, cc);
+    load8_f32(sinT + trow * 64 + g * 8, ss);
     const float sign = (g & 2) ? 1.f : -1.f;
     float o[8];
 #pragma unroll
@@ -394,18 +397,41 @@ extern "C" int fwb_ln_modulate(const void* x, int x_dtype, int64_t ldx, int rows
   return FWB_OK;
 }
 
-extern "C" int fwb_rmsnorm_rope(void* x, int64_t ldx, int rows, int C, const float* w, float eps, const float* cos_sin,
-                                int head_dim, cudaStream_t stream) {
+extern "C" int fwb_rmsnorm_rope_periodic(void* x, int64_t ldx, int rows, int C, const float* w, float eps, const float* cos_sin,
+                                         int table_rows, int head_dim, cudaStream_t stream) {
   FWB_CHECK(x, "rmsnorm_rope: null pointer");
   FWB_CHECK(rows > 0 && C > 0, "rmsnorm_rope: empty problem");
   FWB_CHECK(C % 8 == 0 && C <= 5120 && ldx % 8 == 0, "rmsnorm_rope: C=%d must be a multiple of 8 and <= 5120", C);
   FWB_CHECK(!cos_sin || (head_dim > 0 && head_dim % 8 == 0 && C % head_dim == 0), "rmsnorm_rope: bad head_dim %d", head_dim);
+  FWB_CHECK(!cos_sin || (table_rows > 0 && rows % table_rows == 0),
+            "rmsnorm_rope: table_rows=%d must divide rows=%d", table_rows, rows);
+  if (!cos_sin) table_rows = 1;
   const int chunks = (C / 8 + kRowThreads - 1) / kRowThreads;
   __nv_bfloat16* xp = reinterpret_cast<__nv_bfloat16*>(x);
   const float2* cs = reinterpret_cast<const float2*>(cos_sin);
-  if (chunks <= 1) rmsnorm_rope_kernel<1><<<row_grid<rmsnorm_rope_kernel<1>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, head_dim);
-  else if (chunks <= 2) rmsnorm_rope_kernel<2><<<row_grid<rmsnorm_rope_kernel<2>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, head_dim);
-  else rmsnorm_rope_kernel<5><<<row_grid<rmsnorm_rope_kernel<5>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, head_dim);
+  if (chunks <= 1) rmsnorm_rope_kernel<1><<<row_grid<rmsnorm_rope_kernel<1>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, table_rows, head_dim);
+  else if (chunks <= 2) rmsnorm_rope_kernel<2><<<row_grid<rmsnorm_rope_kernel<2>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, table_rows, head_dim);
+  else rmsnorm_rope_kernel<5><<<row_grid<rmsnorm_rope_kernel<5>>(rows), kRowThreads, 0, stream>>>(xp, ldx, rows, C, w, eps, cs, table_rows, head_dim);
+  FWB_CUDA(cudaGetLastError());
+  return FWB_OK;
+}
+
+extern "C" int fwb_rmsnorm_rope(void* x, int64_t ldx, int rows, int C, const float* w, float eps, const float* cos_sin,
+                                int head_dim, cudaStream_t stream) {
+  return fwb_rmsnorm_rope_periodic(x, ldx, rows, C, w, eps, cos_sin, rows, head_dim, stream);
+}
+
+extern "C" int fwb_ln64_rope2d_periodic(void* qkv, int64_t ld, int rows, int H, float eps, const float* qw, const float* qb,
+                                        const float* kw, const float* kb, const float* cosT, const float* sinT, int table_rows,
+                                        cudaStream_t stream) {
+  FWB_CHECK(qkv && qw && qb && kw && kb && cosT && sinT, "ln64_rope2d: null pointer");
+  FWB_CHECK(rows > 0 && H > 0 && ld % 8 == 0 && ld >= 3LL * H * 64, "ln64_rope2d: bad shape rows=%d H=%d ld=%lld", rows, H, (long long)ld);
+  FWB_CHECK(table_rows > 0 && rows % table_rows == 0, "ln64_rope2d: table_rows=%d must divide rows=%d", table_rows, rows);
+  const long long threads = (long long)rows * 2 * H * 8;
+  const long long blocks = (threads + 255) / 256;
+  FWB_CHECK(blocks < 2147483647LL, "ln64_rope2d: too many rows");
+  ln64_rope2d_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<__nv_bfloat16*>(qkv), ld, rows, H, eps, qw, qb,
+                                                         kw, kb, cosT, sinT, table_rows);
   FWB_CUDA(cudaGetLastError());
   return FWB_OK;
 }
@@ -413,15 +439,7 @@ extern "C" int fwb_rmsnorm_rope(void* x, int64_t ldx, int rows, int C, const flo
 extern "C" int fwb_ln64_rope2d(void* qkv, int64_t ld, int rows, int H, float eps, const float* qw, const float* qb,
                                const float* kw, const float* kb, const float* cosT, const float* sinT,
                                cudaStream_t stream) {
-  FWB_CHECK(qkv && qw && qb && kw && kb && cosT && sinT, "ln64_rope2d: null pointer");
-  FWB_CHECK(rows > 0 && H > 0 && ld % 8 == 0 && ld >= 3LL * H * 64, "ln64_rope2d: bad shape rows=%d H=%d ld=%lld", rows, H, (long long)ld);
-  const long long threads = (long long)rows * 2 * H * 8;
-  const long long blocks = (threads + 255) / 256;
-  FWB_CHECK(blocks < 2147483647LL, "ln64_rope2d: too many rows");
-  ln64_rope2d_kernel<<<(unsigned)blocks, 256, 0, stream>>>(reinterpret_cast<__nv_bfloat16*>(qkv), ld, rows, H, eps, qw, qb,
-                                                         kw, kb, cosT, sinT);
-  FWB_CUDA(cudaGetLastError());
-  return FWB_OK;
+  return fwb_ln64_rope2d_periodic(qkv, ld, rows, H, eps, qw, qb, kw, kb, cosT, sinT, rows, stream);
 }
 
 extern "C" int fwb_cfg_euler_step(void* latents, const void* pred_pos, const void* pred_neg, int64_t n, float cfg_scale,

@@ -65,7 +65,9 @@ def _load():
     lib.fwb_rowwise_set_ctas_per_sm.argtypes = [i32]
     lib.fwb_ln_modulate.argtypes = [vp, i32, i64, i32, i32, f32, vp, vp, vp, vp, vp, i64, vp]
     lib.fwb_rmsnorm_rope.argtypes = [vp, i64, i32, i32, vp, f32, vp, i32, vp]
+    lib.fwb_rmsnorm_rope_periodic.argtypes = [vp, i64, i32, i32, vp, f32, vp, i32, i32, vp]
     lib.fwb_ln64_rope2d.argtypes = [vp, i64, i32, i32, f32, vp, vp, vp, vp, vp, vp, vp]
+    lib.fwb_ln64_rope2d_periodic.argtypes = [vp, i64, i32, i32, f32, vp, vp, vp, vp, vp, vp, i32, vp]
     lib.fwb_cfg_euler_step.argtypes = [vp, vp, vp, i64, f32, f32, vp]
     for name in abi_symbols():
         fn = getattr(lib, name)  # raises AttributeError if a declared symbol is not exported

@@ -142,11 +142,18 @@ def rope2d_expanded(pos: torch.Tensor, base: float = 100.0):
     i.e. INSIDE the sampler's `torch.cuda.amp.autocast(bf16)` region (inference_wan21.py:310), where einsum is an
     autocast-to-bf16 op: angle = bf16(bf16(pos) * bf16(inv_freq)), then cos/sin in fp32.  That is what the released
     weights were trained and are run with, so it is reproduced here explicitly (independent of any ambient autocast).
-    FWB_ROPE2D_FP32_ANGLES=1 (or engine.ROPE2D_FP32_ANGLES = True) selects the reference's no-autocast (fp32) arithmetic."""
+    FWB_ROPE2D_FP32_ANGLES=1 (or engine.ROPE2D_FP32_ANGLES = True) selects the reference's no-autocast (fp32) arithmetic.
+
+    A position tensor whose base carries `_fwb_period` (Aggregator._positions at batch > 1: every sample has the same
+    positions) gets tables of that many rows only; ops.ln64_rope2d_ applies them periodically."""
     fp32_angles = ROPE2D_FP32_ANGLES
+    base_t = pos._base if pos._base is not None else pos   # views of one position tensor share the tables
+    period = getattr(base_t, "_fwb_period", None)
 
     def build():
         p = pos.reshape(-1, 2).long()
+        if period is not None:
+            p = p[:period]
         dim = 32
         with torch.autocast(device_type=p.device.type, enabled=False):
             exponents = torch.arange(0, dim, 2, device=p.device).float() / dim
@@ -163,26 +170,56 @@ def rope2d_expanded(pos: torch.Tensor, base: float = 100.0):
             sinT = torch.cat([sin_t[p[:, 0]], sin_t[p[:, 1]]], dim=-1).contiguous()
         return cosT, sinT
 
-    base_t = pos._base if pos._base is not None else pos   # views of one position tensor share the tables
-    return _r2d_cache.get((base_t,), (pos.numel(), base, fp32_angles), build)
+    return _r2d_cache.get((base_t,), (pos.numel(), base, fp32_angles, period), build)
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# batch: every sample of a call shares the timestep
+# ------------------------------------------------------------------------------------------------------------------
+SHARED_TIMESTEP_MSG = ("samples of one batch must share the timestep: the reference's joint_forward has no per-sample "
+                       "timestep semantics (at timesteps [900, 500] its batch-2 outputs differ from its own batch-1 runs by up to 1.46)")
+
+
+def shared_timestep(timestep: torch.Tensor, batch: int) -> torch.Tensor:
+    """Validate the timestep of a batch-`batch` call and return it as one element ([1]).  A timestep with 1 element, or with
+    `batch` equal elements, is accepted; anything else raises ValueError.  Pure tensor logic, checked before any launch."""
+    t = timestep.reshape(-1)
+    if t.numel() not in (1, batch):
+        raise ValueError(f"timestep has {t.numel()} elements for a batch of {batch}: give 1, or {batch} equal values")
+    if t.numel() > 1 and not bool((t == t[:1]).all()):
+        raise ValueError(SHARED_TIMESTEP_MSG + f"; got {t.tolist()}")
+    return t[:1]
+
+
+def shared_rows(m: torch.Tensor, what: str) -> torch.Tensor:
+    """m [B, ...] -> m[:1] when all B rows are equal (a shared timestep), else ValueError.  B == 1 is returned as is."""
+    if m.shape[0] > 1 and not bool((m == m[:1]).all()):
+        raise ValueError(f"{what}: " + SHARED_TIMESTEP_MSG)
+    return m[:1]
+
+
+def _heads(t, B, H, D):
+    """[B*L, H*D] row view -> [B, L, H, D] view (no copy)."""
+    return t.unflatten(1, (H, D)).unflatten(0, (B, -1))
 
 
 # ------------------------------------------------------------------------------------------------------------------
 # DiT block pieces (reference: diffsynth_wan21/models/wan_video_dit.py DiTBlock / SelfAttention / CrossAttention)
 # ------------------------------------------------------------------------------------------------------------------
 def dit_mod_vectors(block, t_mod):
-    """(modulation + t_mod).chunk(6) as fp32 vectors: shift, (1+scale) [rounded to bf16 first], gate — twice."""
-    m = (block.modulation.to(BF16) + t_mod.to(BF16))  # [1, 6, C] bf16 add, as under autocast
-    assert m.shape[0] == 1, "fused path handles batch 1 (the reference sampler's batch)"
+    """(modulation + t_mod).chunk(6) as fp32 vectors: shift, (1+scale) [rounded to bf16 first], gate — twice.
+    t_mod [B, 6, C] must have equal rows (shared timestep, see shared_timestep)."""
+    m = shared_rows(block.modulation.to(BF16) + t_mod.to(BF16), "dit_mod_vectors")  # [1, 6, C] bf16 add, as under autocast
     one_plus = (1 + m[0, [1, 4]]).float()              # bf16(1 + scale)
     mf = m[0].float()
     return dict(shift_msa=mf[0].contiguous(), mul_msa=one_plus[0].contiguous(), gate_msa=mf[2].contiguous(),
                 shift_mlp=mf[3].contiguous(), mul_mlp=one_plus[1].contiguous(), gate_mlp=mf[5].contiguous())
 
 
-def dit_self_attn(sa, h, cos_sin, x_resid, gate):
-    """x_resid + gate * o(attn(rope(norm_q(q(h))), rope(norm_k(k(h))), v(h)))  — wan_video_dit.py:175-182, 301."""
-    L = h.shape[0]
+def dit_self_attn(sa, h, cos_sin, x_resid, gate, n_batch=1):
+    """x_resid + gate * o(attn(rope(norm_q(q(h))), rope(norm_k(k(h))), v(h)))  — wan_video_dit.py:175-182, 301.
+    h [n_batch * L, C]: each sample attends over its own L tokens; cos_sin holds the L per-position rows."""
+    rows = h.shape[0]
     H, D = sa.num_heads, sa.head_dim
     C = H * D
     if SP is None:
@@ -191,10 +228,11 @@ def dit_self_attn(sa, h, cos_sin, x_resid, gate):
         v = lin(h, sa.v)
         ops.rmsnorm_rope_(q, w=f32(sa.norm_q, "w", sa.norm_q.weight), eps=sa.norm_q.eps, cos_sin=cos_sin, head_dim=D)
         ops.rmsnorm_rope_(k, w=f32(sa.norm_k, "w", sa.norm_k.weight), eps=sa.norm_k.eps, cos_sin=cos_sin, head_dim=D)
-        o = ops.attention(q.view(1, L, H, D), k.view(1, L, H, D), v.view(1, L, H, D))
+        o = ops.attention(_heads(q, n_batch, H, D), _heads(k, n_batch, H, D), _heads(v, n_batch, H, D))
     else:
         # sequence parallel: h holds this rank's L/P tokens.  K and V are written side by side into one packed buffer so
         # that a single exchange moves both; queries stay local.
+        L = rows
         kv = torch.empty((L, 2 * C), device=h.device, dtype=BF16)
         lin(h, sa.k, out=kv[:, :C])
         lin(h, sa.v, out=kv[:, C:])
@@ -223,32 +261,35 @@ def dit_self_attn(sa, h, cos_sin, x_resid, gate):
                 main.wait_event(ev)
                 ops.attention_partial(q4, heads(buf[:, :C]), heads(buf[:, C:]), part[c], lse[c])
             o = ops.attention_merge(part, lse)
-    return lin(o.view(L, C), sa.o, scale1=gate, resid=x_resid, round_flags=ROUND_AFTER_BIAS | ROUND_AFTER_AFFINE)
+    return lin(o.view(rows, C), sa.o, scale1=gate, resid=x_resid, round_flags=ROUND_AFTER_BIAS | ROUND_AFTER_AFFINE)
 
 
 def cross_kv(ca, context):
-    """Loop-invariant K/V of the text / CLIP context (SURVEY Appendix E) — cached per context tensor."""
+    """Loop-invariant K/V of the text / CLIP context (SURVEY Appendix E) — cached per context tensor.
+    context [B, n_ctx, C] -> per-sample K/V [B, n, H, D] (text, then CLIP or None)."""
     cache = ca.__dict__.get("_fwb_kv")
     if cache is None:
         cache = ca.__dict__["_fwb_kv"] = IdCache(4)
 
     def build():
         ctx = as_bf16(context)
-        assert ctx.shape[0] == 1
+        B, C = ctx.shape[0], ctx.shape[-1]
         H, D = ca.num_heads, ca.head_dim
         if ca.has_image_input:
-            img, txt = ctx[0, :257], ctx[0, 257:]
+            img, txt = ctx[:, :257], ctx[:, 257:]
         else:
-            img, txt = None, ctx[0]
-        k = lin(txt.contiguous(), ca.k)
+            img, txt = None, ctx
+        txt = txt.reshape(-1, C).contiguous()
+        k = lin(txt, ca.k)
         ops.rmsnorm_rope_(k, w=f32(ca.norm_k, "w", ca.norm_k.weight), eps=ca.norm_k.eps)
-        v = lin(txt.contiguous(), ca.v)
-        out = [k.view(1, -1, H, D), v.view(1, -1, H, D), None, None]
+        v = lin(txt, ca.v)
+        out = [k.view(B, -1, H, D), v.view(B, -1, H, D), None, None]
         if img is not None:
-            ki = lin(img.contiguous(), ca.k_img)
+            img = img.reshape(-1, C).contiguous()
+            ki = lin(img, ca.k_img)
             ops.rmsnorm_rope_(ki, w=f32(ca.norm_k_img, "w", ca.norm_k_img.weight), eps=ca.norm_k_img.eps)
-            vi = lin(img.contiguous(), ca.v_img)
-            out[2], out[3] = ki.view(1, -1, H, D), vi.view(1, -1, H, D)
+            vi = lin(img, ca.v_img)
+            out[2], out[3] = ki.view(B, -1, H, D), vi.view(B, -1, H, D)
         return out
 
     srcs = (context, ca.k.weight, ca.v.weight)
@@ -256,17 +297,20 @@ def cross_kv(ca, context):
 
 
 def dit_cross_attn_core(ca, n3, context):
-    """q-projection + text attention (+ CLIP attention, summed in bf16) — wan_video_dit.py:185-201.  Returns [L, C]."""
-    L = n3.shape[0]
+    """q-projection + text attention (+ CLIP attention, summed in bf16) — wan_video_dit.py:185-201.  n3 [B * L, C] against the
+    context of each sample ([B, n_ctx, C]).  Returns [B * L, C]."""
+    rows = n3.shape[0]
     H, D = ca.num_heads, ca.head_dim
     k, v, ki, vi = cross_kv(ca, context)
+    if rows % k.shape[0]:
+        raise ValueError(f"cross attention: {rows} query rows do not split over a context batch of {k.shape[0]}")
     q = lin(n3, ca.q)
     ops.rmsnorm_rope_(q, w=f32(ca.norm_q, "w", ca.norm_q.weight), eps=ca.norm_q.eps)
-    q4 = q.view(1, L, H, D)
+    q4 = _heads(q, k.shape[0], H, D)
     o = ops.attention(q4, k, v)
     if ki is not None:
         ops.attention(q4, ki, vi, out=o, accumulate=True)
-    return o.view(L, H * D)
+    return o.view(rows, H * D)
 
 
 def dit_ffn(block, x, mods):
@@ -280,9 +324,9 @@ def dit_ffn(block, x, mods):
 # VGGT block pieces (reference: vggt/layers/block.py Block, vggt/layers/attention.py Attention)
 # ------------------------------------------------------------------------------------------------------------------
 def vggt_mod_vectors(block, e0):
-    """(modulation + e0).chunk(6) in fp32 — vggt/layers/block.py:95-104 (batch 1)."""
-    assert e0 is not None and e0.shape[0] == 1
-    e = (block.modulation.float() + e0.float())[0]  # [6, C]
+    """(modulation + e0).chunk(6) in fp32 — vggt/layers/block.py:95-104.  e0 [B, 6, C] must have equal rows (shared timestep)."""
+    assert e0 is not None
+    e = shared_rows(block.modulation.float() + e0.float(), "vggt_mod_vectors")[0]  # [6, C]
     return dict(add1=e[0].contiguous(), mul1=(1 + e[1]).contiguous(), add2=e[3].contiguous(),
                 mul2=(1 + e[4]).contiguous(), e5=e[5].contiguous())
 
@@ -331,8 +375,9 @@ def vggt_ffn_part(block, x, mods):
 # ------------------------------------------------------------------------------------------------------------------
 # bidirectional adapter (reference: fusion/layer/block.py CrossModalityBiAttentionBlock / BiMultiHeadAttention)
 # ------------------------------------------------------------------------------------------------------------------
-def bicross(blk, x1, x2, cs_dit, cs_agg):
-    """x1 [L1, C1] bf16 (video), x2 [L2, C2] fp32|bf16 (geometry) -> updated (x1, x2)."""
+def bicross(blk, x1, x2, cs_dit, cs_agg, n_batch=1):
+    """x1 [B*L1, C1] bf16 (video), x2 [B*L2, C2] fp32|bf16 (geometry) -> updated (x1, x2); sample b's video tokens attend to
+    sample b's geometry tokens and back.  cs_dit / cs_agg hold the L1 / L2 per-position rows."""
     ca = blk.cross_attn
     H, D, E = ca.num_heads, ca.head_dim, ca.embed_dim
     L1, L2 = x1.shape[0], x2.shape[0]
@@ -347,10 +392,10 @@ def bicross(blk, x1, x2, cs_dit, cs_agg):
     kv2 = ops.linear(n2, w2, bias=b2)
     ops.rmsnorm_rope_(qv1[:, :E], cos_sin=cs_dit, head_dim=D)
     ops.rmsnorm_rope_(kv2[:, :E], cos_sin=cs_agg, head_dim=D)
-    q = qv1[:, :E].unflatten(1, (H, D)).unsqueeze(0)
-    v1 = qv1[:, E:].unflatten(1, (H, D)).unsqueeze(0)
-    k = kv2[:, :E].unflatten(1, (H, D)).unsqueeze(0)
-    v2 = kv2[:, E:].unflatten(1, (H, D)).unsqueeze(0)
+    q = _heads(qv1[:, :E], n_batch, H, D)
+    v1 = _heads(qv1[:, E:], n_batch, H, D)
+    k = _heads(kv2[:, :E], n_batch, H, D)
+    v2 = _heads(kv2[:, E:], n_batch, H, D)
     if SP is None:
         o1 = ops.attention(q, k, v2)   # video <- geometry
         o2 = ops.attention(k, q, v1)   # geometry <- video

@@ -285,29 +285,40 @@ def ln_modulate(x: torch.Tensor, *, eps: float, w=None, b=None, mul=None, add=No
 
 
 def rmsnorm_rope_(x: torch.Tensor, *, w=None, eps: float = 1e-6, cos_sin=None, head_dim: int = 0) -> torch.Tensor:
-    """In place on bf16 x [rows, C] (row stride allowed): full-row RMSNorm(+w) then interleaved-pair RoPE."""
+    """In place on bf16 x [rows, C] (row stride allowed): full-row RMSNorm(+w) then interleaved-pair RoPE.  cos_sin
+    [T, head_dim/2, 2] with T dividing rows: row r uses table row r % T (a batch of B samples shares one per-position table)."""
     assert x.dim() == 2 and x.stride(1) == 1 and x.dtype == torch.bfloat16 and x.is_cuda
     rows, C = x.shape
+    table_rows = rows
     if cos_sin is not None:
-        assert cos_sin.dtype == torch.float32 and cos_sin.is_contiguous() and cos_sin.shape == (rows, head_dim // 2, 2)
+        table_rows = cos_sin.shape[0]
+        assert cos_sin.dtype == torch.float32 and cos_sin.is_contiguous() and cos_sin.shape[1:] == (head_dim // 2, 2)
+        if rows % table_rows:
+            raise ValueError(f"rmsnorm_rope_: RoPE table of {table_rows} rows does not divide {rows} token rows")
     _count()
     with _Rec(f"rmsrope:R{rows}:C{C}"):
-      check(lib.fwb_rmsnorm_rope(x.data_ptr(), x.stride(0), rows, C, _vec(w, C, "w"), float(eps),
-                               None if cos_sin is None else cos_sin.data_ptr(), head_dim, _stream()), "fwb_rmsnorm_rope")
+      check(lib.fwb_rmsnorm_rope_periodic(x.data_ptr(), x.stride(0), rows, C, _vec(w, C, "w"), float(eps),
+                                        None if cos_sin is None else cos_sin.data_ptr(), table_rows, head_dim, _stream()),
+            "fwb_rmsnorm_rope_periodic")
     _nan_check(f"rmsrope:R{rows}:C{C}", x)
     return x
 
 
 def ln64_rope2d_(qkv: torch.Tensor, H: int, *, eps: float, qw, qb, kw, kb, cosT, sinT) -> torch.Tensor:
-    """In place on packed qkv bf16 [rows, 3*H*64]: per-head LayerNorm + 2-D RoPE on the q and k thirds."""
+    """In place on packed qkv bf16 [rows, 3*H*64]: per-head LayerNorm + 2-D RoPE on the q and k thirds.  cosT / sinT [T, 64]
+    with T dividing rows: row r uses table row r % T."""
     assert qkv.dim() == 2 and qkv.stride(1) == 1 and qkv.dtype == torch.bfloat16 and qkv.is_cuda
     rows = qkv.shape[0]
-    assert cosT.shape == (rows, 64) and sinT.shape == (rows, 64) and cosT.is_contiguous() and sinT.is_contiguous()
+    table_rows = cosT.shape[0]
+    assert cosT.shape == (table_rows, 64) and sinT.shape == (table_rows, 64) and cosT.is_contiguous() and sinT.is_contiguous()
+    if rows % table_rows:
+        raise ValueError(f"ln64_rope2d_: RoPE table of {table_rows} rows does not divide {rows} token rows")
     _count()
     with _Rec(f"ln64rope:R{rows}:H{H}"):
-      check(lib.fwb_ln64_rope2d(qkv.data_ptr(), qkv.stride(0), rows, H, float(eps), _vec(qw, 64, "qw"), _vec(qb, 64, "qb"),
-                              _vec(kw, 64, "kw"), _vec(kb, 64, "kb"), cosT.data_ptr(), sinT.data_ptr(), _stream()),
-          "fwb_ln64_rope2d")
+      check(lib.fwb_ln64_rope2d_periodic(qkv.data_ptr(), qkv.stride(0), rows, H, float(eps), _vec(qw, 64, "qw"), _vec(qb, 64, "qb"),
+                                       _vec(kw, 64, "kw"), _vec(kb, 64, "kb"), cosT.data_ptr(), sinT.data_ptr(), table_rows,
+                                       _stream()),
+          "fwb_ln64_rope2d_periodic")
     _nan_check(f"ln64rope:R{rows}", qkv)
     return qkv
 

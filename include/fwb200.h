@@ -157,12 +157,25 @@ int fwb_rowwise_set_ctas_per_sm(int n);
  *           (DiT :178-179; adapter fusion/layer/block.py:545-550). */
 int fwb_rmsnorm_rope(void* x, int64_t ldx, int rows, int C, const float* w, float eps, const float* cos_sin, int head_dim,
                      fwb_stream_t stream);
+/* Batched form: row r reads cos_sin row (r % table_rows); table_rows must divide rows.  At batch B the token rows are B*L
+ * while the table is per position (L rows), so one cached table serves every sample.  fwb_rmsnorm_rope is this call with
+ * table_rows = rows (same results).
+ * Call sites: the DiT self-attention q/k (wan_video_dit.py:176-179) and the adapter q/k (fusion/layer/block.py:545-550)
+ * at batch > 1 (fwb200/engine.py dit_self_attn, bicross). */
+int fwb_rmsnorm_rope_periodic(void* x, int64_t ldx, int rows, int C, const float* w, float eps, const float* cos_sin,
+                              int table_rows, int head_dim, fwb_stream_t stream);
 
 /* ---- K8+K9 (VGGT): per-head LayerNorm(64) + 2-D rotate-half RoPE on q and k of a packed qkv buffer, in place --------
  * qkv: bf16 [rows, 3*H*64] laid out (3, H, 64); cosT/sinT: fp32 [rows, 64] expanded tables (first 32 = y, last 32 = x).
  * Replaces: q_norm/k_norm + rope vggt/layers/attention.py:52-58, vggt/layers/rope.py:133-188. */
 int fwb_ln64_rope2d(void* qkv, int64_t ld, int rows, int H, float eps, const float* qw, const float* qb, const float* kw,
                     const float* kb, const float* cosT, const float* sinT, fwb_stream_t stream);
+/* Batched form: row r reads cosT / sinT row (r % table_rows); table_rows must divide rows.  fwb_ln64_rope2d is this call with
+ * table_rows = rows (same results).
+ * Call sites: the VGGT frame and global blocks (vggt/layers/attention.py:52-58) at batch > 1, where the positions of every
+ * sample are the same (fwb200/engine.py vggt_attn_part, tables from FantasyWorld/vggt/models/aggregator.py _positions). */
+int fwb_ln64_rope2d_periodic(void* qkv, int64_t ld, int rows, int H, float eps, const float* qw, const float* qb, const float* kw,
+                             const float* kb, const float* cosT, const float* sinT, int table_rows, fwb_stream_t stream);
 
 /* ---- a1/a18: classifier-free guidance + flow-matching Euler update, in place on bf16 latents ------------------------
  * latents <- latents + (neg + cfg*(pos-neg)) * dsigma with the reference's bf16 rounding after every op.
